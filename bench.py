@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — mesh-tokens/sec of the auto-regressive decode hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--max-new T] [--workload decode|tf|dit|train]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--max-new T] [--workload decode|tf|dit|train] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, replicas)
 
 A "step" is one complete pass of the hot path over one synthetic request of BASELINE.json configs[1]:
@@ -20,6 +20,7 @@ that copy is absent, the CPU oracle port (kind "port").  reference_gpu = the sam
 """
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -60,6 +61,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(['nvidia-smi', '-i', str(self.index), '--query-gpu=' + q, '--format=csv,noheader,nounits', '-lms', '200'],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)                     # no sampler left running if the benchmark fails before stop()
             self.thread = threading.Thread(target=lambda: [self.lines.append(l) for l in self.proc.stdout], daemon=True)
             self.thread.start()
         except Exception:
@@ -88,6 +90,24 @@ class ClockSampler:
                     reasons.add(n)
         return {'sm_mhz': float(np.median(sm)) if sm else None, 'sm_max_mhz': max(mx) if mx else None,
                 'reasons': sorted(reasons), 'samples': len(sm)}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: what the timed path returned in its last step, one <path>/<name>.npy per array in float64.  An array larger than its
+    share of DUMP_BYTES is replaced by a fixed, seeded sample of its flattened elements, and <name>_index.npy holds their flat indices.
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // (2 * len(arrays))
+    for name, a in arrays.items():
+        a = torch.as_tensor(a).detach()
+        if a.numel() * 8 > share:                           # sampled where the array lives: no float64 copy of it on the host
+            idx = np.sort(np.random.default_rng(0).choice(a.numel(), share // 8, replace=False))
+            np.save(os.path.join(path, name + '_index.npy'), idx.astype(np.float64))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(path, name + '.npy'), a.cpu().numpy().astype(np.float64))
 
 
 def algorithmic_decode_bytes(eng, L0, T):
@@ -283,6 +303,8 @@ def run_teacher_forced(args):
     ev[1].record()
     barrier()
     ms = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     if world > 1:
         import torch.distributed as dist
         t = torch.tensor([ms, comm_ms or 0.0], dtype=torch.float64, device=dev)
@@ -377,6 +399,9 @@ def run_train(args):
     ev[1].record()
     barrier()
     ms = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:
+        # the step's losses and gradient norm, and the updated fp32 parameters it leaves in the trainer
+        dump_outputs(args.dump_outputs, {**{k: out[k] for k in ('loss', 'loss_ce', 'loss_kl', 'grad_norm')}, 'parameters': tr.param})
     if world > 1:
         import torch.distributed as dist
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -518,6 +543,8 @@ def run_dit(args):
     barrier()
     launches = eng.kernel_launches() - l0
     ms = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'latents': lat})
     # e2e: host buffers through the C ABI
     lat_h = np.empty_like(noise_h.numpy())
     e2e_steps = max(1, min(args.steps, args.e2e_steps))
@@ -680,7 +707,13 @@ def main():
                     help="decode = BASELINE configs[1] (the metric); tf = configs[3]: teacher-forced forward seq 8192 batch 4/GPU, loss all-reduced over NCCL")
     ap.add_argument('--freeze-encoder', action='store_true', help='--workload train: opt.freeze_encoder = True (the Options default) instead of the ArAE preset (encoder trained)')
     ap.add_argument('--debug', action='append', default=[], metavar='KEY=VALUE', help='process-wide experiment switch of the library (er_debug_set(NULL, KEY, VALUE)), e.g. attn_bwd_wmma=1')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last one computed to DIR/<name>.npy (float64, '
+                    'at most 64 MB in all; seeded inputs, so two builds can be compared output for output)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs records the CUDA path; the reference arm has none')
     # stdout carries exactly ONE JSON line: whatever libraries print there (NCCL's version banner under torchrun) is sent to stderr instead
     global _STDOUT_FD
     sys.stdout.flush()
@@ -761,7 +794,6 @@ def main():
     for _ in range(args.warmup):
         out = step_device()
     barrier()
-    n_tok = int(out['n'].item())
     launches0 = eng.kernel_launches()
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -778,6 +810,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     launches = eng.kernel_launches() - launches0
     n_tok = int(out['n'].item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'tokens': out['ids'][:n_tok]})
     value = world * args.steps * n_tok / (ms_total / 1e3)
     dec_ms_avg = float(np.mean(dec_ms))
 

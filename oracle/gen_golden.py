@@ -434,6 +434,35 @@ def gen_meto_clers_goldens():
     print('[gen] wrote meto_clers.npz', len(names), 'meshes', len(streams), 'streams', flush=True)
 
 
+def gen_meto_live_goldens():
+    """The compiled reference's Engine_LR_ABSCO / Engine_LR on meshes.random_grids(): encode, then decode of its own tokens.  Each field
+    of all encodings is stored concatenated (in the dtype that holds it exactly: the decoded vertices are fp32 values) with a length per
+    encoding, in iteration order, LR_ABSCO before LR."""
+    import _meto
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    import meshes
+    fields = {'tokens': np.int16, 'order': np.int16, 'ftype': np.int8, 'dv': np.float32, 'df': np.int16, 'dt': np.int8}
+    parts = {k: [] for k in fields}
+    bins_all = []
+    for it, v, f, bins in meshes.random_grids():
+        for ref_cls in (_meto.Engine_LR_ABSCO, _meto.Engine_LR):
+            ref = ref_cls(bins, False)
+            tok, order, ftype = ref.encode(v.tolist(), f.tolist())
+            dv, df, dt = ref.decode(tok)
+            got = {'tokens': tok, 'order': order, 'ftype': ftype, 'dv': np.reshape(dv, (-1, 3)), 'df': np.reshape(df, (-1, 3)), 'dt': dt}
+            for k, dtype in fields.items():
+                a = np.asarray(got[k])
+                assert np.array_equal(a.astype(dtype), a), k
+                parts[k].append(a.astype(dtype))
+            bins_all.append(bins)
+    out = {'bins': np.asarray(bins_all, dtype=np.int32)}
+    for k, p in parts.items():
+        out[k] = np.concatenate(p)
+        out['n_' + k] = np.asarray([len(x) for x in p], dtype=np.int32)
+    np.savez_compressed(os.path.join(GOLD, 'meto_live.npz'), **out)
+    print('[gen] wrote meto_live.npz', len(bins_all), 'encodings', flush=True)
+
+
 def gen_dit_goldens():
     """The reference DiT module itself (core/transformer/dit.py), CPU fp32, naive attention, on the seeded weights of oracle/dit_oracle.py."""
     from core.transformer.dit import DiT
@@ -527,6 +556,8 @@ def main():
         gen_meto_goldens()
     if args.only in ('all', 'meto_clers'):
         gen_meto_clers_goldens()
+    if args.only in ('all', 'meto_live'):
+        gen_meto_live_goldens()
     if args.only in ('all', 'dit'):
         gen_dit_goldens()
     if args.only in ('all', 'provider'):

@@ -1,5 +1,5 @@
-import ctypes as C, sys
-sys.path.insert(0,'/root/repo')
+import ctypes as C, os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from edgerunner_b200 import _lib
 lib = C.CDLL(_lib.LIB_PATH)

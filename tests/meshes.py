@@ -181,3 +181,22 @@ def stress_meshes(count=24):
             f = f[r.rand(len(f)) > 0.05]
         out[f'stress{seed}'] = (np.ascontiguousarray(v, dtype=np.float32), np.ascontiguousarray(f, dtype=np.int32))
     return out
+
+
+def random_grids(count=40, seed=2024):
+    """Jittered grids with holes, flipped and shuffled faces (every fifth with extra random faces), each with a random bin count:
+    yields (index, vertices, faces, bins).  Deterministic for a given seed."""
+    rng = np.random.RandomState(seed)
+    for it in range(count):
+        nx, ny = rng.randint(2, 14, size=2)
+        v, f = grid(int(nx), int(ny))
+        v = v + rng.uniform(-0.03, 0.03, v.shape).astype(np.float32)
+        f = f[rng.rand(len(f)) > rng.uniform(0, 0.3)]
+        fl = rng.rand(len(f)) < rng.uniform(0, 0.5)
+        f[fl] = f[fl][:, ::-1]
+        f = f[rng.permutation(len(f))]
+        if it % 5 == 0:                                     # some outright garbage connectivity
+            f = np.concatenate([f, rng.randint(0, len(v), (7, 3)).astype(np.int32)])
+        v = np.clip(v, -1, 1)
+        bins = int(rng.choice([4, 32, 256, 512, 1024]))
+        yield it, v, f, bins

@@ -26,6 +26,27 @@ def test_reference_arm_json_line():
     assert d['value'] > 0 and 'workload' in d['config']
 
 
+def test_dump_outputs_budget_and_sample(tmp_path):
+    """--dump-outputs: every array in float64; one above its share of the 64 MB budget becomes a fixed seeded sample plus its indices."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, REPO)
+    import bench
+    arrays = {'loss': torch.tensor(1.5), 'tokens': torch.arange(7, dtype=torch.int32), 'logits': torch.arange(6_000_000, dtype=torch.float32).reshape(1000, 6000)}
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / 'a'))
+    assert files == ['logits.npy', 'logits_index.npy', 'loss.npy', 'tokens.npy']
+    got = {f: np.load(tmp_path / 'a' / f) for f in files}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in files) <= bench.DUMP_BYTES
+    assert got['loss.npy'] == 1.5 and np.array_equal(got['tokens.npy'], np.arange(7))
+    idx = got['logits_index.npy']
+    assert 0 < len(idx) < 6_000_000 and np.all(np.diff(idx) > 0) and np.array_equal(got['logits.npy'], idx)
+    for f in files:
+        assert np.array_equal(got[f], np.load(tmp_path / 'b' / f)), f
+
+
 def test_algorithmic_byte_model():
     """SURVEY.md §8(d): bytes(L) = W + kv (L + 1) with W = 1,361,504,256 and kv = 147,456 for the ArAE preset; 45.5 TB for the 16k request."""
     sys.path.insert(0, REPO)

@@ -125,45 +125,29 @@ def test_encode_matches_reference_goldens(golden_dir):
     assert n >= 100
 
 
-def test_encode_live_against_compiled_reference():
-    """Fresh random meshes against oracle/_ref/_meto when it is present (built by oracle/Makefile from the reference sources)."""
-    import sys
-    ref_dir = os.path.join(REPO, 'oracle', '_ref')
-    sys.path.insert(0, ref_dir)
-    try:
-        import _meto
-    except ImportError:
-        pytest.skip('compiled reference tokenizer not built (oracle/_ref)')
-    finally:
-        sys.path.remove(ref_dir)
+def test_encode_live_against_compiled_reference(golden_dir):
+    """Random jittered grids (meshes.random_grids) against the compiled reference's Engine_LR_ABSCO / Engine_LR on the same meshes,
+    recorded in meto_live.npz (oracle/gen_golden.py --only meto_live): encode and decode, bit-exact."""
     import meshes
     from meto import Engine
-    rng = np.random.RandomState(2024)
-    for it in range(40):
-        nx, ny = rng.randint(2, 14, size=2)
-        v, f = meshes.grid(int(nx), int(ny))
-        v = v + rng.uniform(-0.03, 0.03, v.shape).astype(np.float32)
-        f = f[rng.rand(len(f)) > rng.uniform(0, 0.3)]
-        fl = rng.rand(len(f)) < rng.uniform(0, 0.5)
-        f[fl] = f[fl][:, ::-1]
-        f = f[rng.permutation(len(f))]
-        if it % 5 == 0:                                     # some outright garbage connectivity
-            f = np.concatenate([f, rng.randint(0, len(v), (7, 3)).astype(np.int32)])
-        v = np.clip(v, -1, 1)
-        bins = int(rng.choice([4, 32, 256, 512, 1024]))
-        for backend, ref_cls in (('LR_ABSCO', _meto.Engine_LR_ABSCO), ('LR', _meto.Engine_LR)):
-            ref = ref_cls(bins, False)
-            rt, ro, rf = ref.encode(v.tolist(), f.tolist())
+    g = np.load(os.path.join(golden_dir, 'meto_live.npz'))
+    ref = {k: np.split(g[k], np.cumsum(g['n_' + k])[:-1]) for k in ('tokens', 'order', 'ftype', 'dv', 'df', 'dt')}
+    n = 0
+    for it, v, f, bins in meshes.random_grids():
+        for backend in ('LR_ABSCO', 'LR'):
+            msg = f'{backend} iter {it}'
+            assert int(g['bins'][n]) == bins, msg
             eng = Engine(bins, backend=backend)
             tok, order, ftype = eng.encode(v, f)
-            np.testing.assert_array_equal(tok, rt, err_msg=f'{backend} iter {it}')
-            np.testing.assert_array_equal(order, ro, err_msg=f'{backend} iter {it}')
-            np.testing.assert_array_equal(ftype, rf, err_msg=f'{backend} iter {it}')
-            dv, df, dt = ref.decode(rt)
+            np.testing.assert_array_equal(tok, ref['tokens'][n], err_msg=msg)
+            np.testing.assert_array_equal(order, ref['order'][n], err_msg=msg)
+            np.testing.assert_array_equal(ftype, ref['ftype'][n], err_msg=msg)
             mv, mf, mt = eng.decode(tok)
-            np.testing.assert_array_equal(mv, np.asarray(dv, dtype=np.float64).reshape(-1, 3), err_msg=f'{backend} iter {it}')
-            np.testing.assert_array_equal(mf, np.asarray(df).reshape(-1, 3), err_msg=f'{backend} iter {it}')
-            np.testing.assert_array_equal(mt, dt, err_msg=f'{backend} iter {it}')
+            np.testing.assert_array_equal(mv, ref['dv'][n].astype(np.float64), err_msg=msg)
+            np.testing.assert_array_equal(mf, ref['df'][n], err_msg=msg)
+            np.testing.assert_array_equal(mt, ref['dt'][n], err_msg=msg)
+            n += 1
+    assert n == len(g['bins']) == 80
 
 
 def test_encode_decode_round_trip():
